@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- BLS12-381 G1 multi-scalar-multiplication throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--logn 20]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--logn 20] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one MSM of 2^logn (scalar, point) pairs (configs[2]: BLS12-381 G1, N = 2^20, uniform 255-bit scalars not
@@ -20,6 +20,8 @@ reduced mod r, points in the prime-order subgroup).  Prints ONE JSON line on ran
   cpu_baseline  the oracle's restatement of the reference's CPU algorithm (kind "port": the Nim reference cannot be
           built in this image) on all host cores, bounded sample.
 --impl reference times that same CPU restatement as the reference arm.
+--dump-outputs DIR writes what the last timed step of each leg returned (dump_outputs), so that two builds can be compared
+          output for output: the inputs depend on the arguments only.
 """
 import argparse
 import ctypes
@@ -33,6 +35,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True           # the benchmark writes nothing into the tree (it may be read-only)
 
 CURVE = "bls12_381_g1"                   # default workload; --curve selects another BASELINE config (same harness)
 INT_MACS_PER_POINT_ADD = 3300            # SURVEY.md 8d: 11 field mults x (2*12^2 + 12) MACs, BLS12-381 G1
@@ -161,8 +164,7 @@ def time_oracle(n_full, budget_s=20.0, max_logn=20):
     from oracle import oracle
     cv = CURVES[CURVE]
     cores = effective_cores()
-    oracle.build()
-    lib = oracle.load()
+    lib = oracle.load()                  # built by __graft_entry__.build(); no rebuild from a possibly read-only tree
     cvt = oracle.curve_t(cv)
     # points for the CPU sample: multiples of G generated by the oracle itself is not needed -- timing does not depend on
     # the values, so reuse a small pool of valid points produced by the exact tier.
@@ -208,6 +210,27 @@ def time_oracle(n_full, budget_s=20.0, max_logn=20):
             "point_adds_per_s": padds / t, "seconds": t, "logn": logn}
 
 
+def dump_outputs(dirname, cv, results):
+    """DIR/msm_<leg>_jac.npy: the Jacobian struct each leg's caller received from its last timed step, as its little-endian 32-bit
+    words (exact in float64), shape (3, words per coordinate), Montgomery form. DIR/msm_resident_affine.npy: that point in affine
+    coordinates, which unlike Jacobian ones are unique, as 32-bit words of the canonical integers, shape (2, extension degree,
+    words per field element); zeros for the point at infinity."""
+    import numpy as np
+    from oracle import pyref
+    os.makedirs(dirname, exist_ok=True)
+    for leg, raw in results.items():
+        words = np.frombuffer(raw[:cv.jac_bytes], dtype="<u4").astype(np.float64).reshape(3, -1)
+        np.save(os.path.join(dirname, f"msm_{leg}_jac.npy"), words)
+    nw = cv.fp.nbytes // 4
+    aff = np.zeros((2, cv.ext_degree, nw), dtype=np.float64)
+    P = pyref.jac_bytes_to_affine(results["resident"], cv)
+    if P is not None:
+        for i, coord in enumerate(P):
+            for j, v in enumerate(coord):
+                aff[i, j] = [(v >> (32 * w)) & 0xFFFFFFFF for w in range(nw)]
+    np.save(os.path.join(dirname, "msm_resident_affine.npy"), aff)
+
+
 def run_reference(args):
     rank, world, local = dist_env()
     if rank != 0:
@@ -242,7 +265,12 @@ def main():
     ap.add_argument("--logn", type=int, default=20)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--curve", default="bls12_381_g1", help="bls12_381_g1 (default, BASELINE metric) | pallas_ec | bls12_381_g2 | ...")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of each leg's last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     global CURVE, INT_MACS_PER_POINT_ADD, ALGO_BYTES_PER_TERM
     CURVE = args.curve
     INT_MACS_PER_POINT_ADD, ALGO_BYTES_PER_TERM = UNIT_FIGURES[CURVE]
@@ -326,6 +354,7 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, steps, warmup, collect=None):
+        """(ms per step on the stream, wall ms per step, what the last step returned)"""
         for _ in range(warmup):
             fn()
         barrier()
@@ -333,7 +362,7 @@ def main():
         t0 = time.perf_counter()
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
             if collect is not None:
                 collect(M.last_stats())
         e1.record()
@@ -346,16 +375,16 @@ def main():
             t = torch.tensor([ms, wall_ms], device=dev, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms, wall_ms = t[0].item(), t[1].item()
-        return ms / steps, wall_ms / steps
+        return ms / steps, wall_ms / steps, last
 
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
     stats = []
-    ms_res, wall_res = timed(step_resident, args.steps, args.warmup, collect=stats.append)
+    ms_res, wall_res, out_res = timed(step_resident, args.steps, args.warmup, collect=stats.append)
     e2e_stats = []
-    ms_e2e, wall_e2e = timed(step_e2e, args.steps, args.warmup, collect=e2e_stats.append)
-    ms_e2e_pg, wall_e2e_pg = timed(step_e2e_pageable, args.steps, args.warmup)
+    ms_e2e, wall_e2e, out_e2e = timed(step_e2e, args.steps, args.warmup, collect=e2e_stats.append)
+    ms_e2e_pg, wall_e2e_pg, out_e2e_pg = timed(step_e2e_pageable, args.steps, args.warmup)
     clocks = sampler.stop() if sampler else None
     # the engine launches strictly in order on one stream, so the CUDA events it records around the accumulation phase bracket
     # those kernels alone
@@ -375,7 +404,7 @@ def main():
             ths = [_th.Thread(target=_worker, args=(2,)) for _ in range(2)]
             [t.start() for t in ths]; [t.join() for t in ths]
         torch.cuda.synchronize()
-        per_thread = max(4, args.steps // 2)
+        per_thread = max(1, args.steps // 2)
         t0 = time.perf_counter()
         ths = [_th.Thread(target=_worker, args=(per_thread,)) for _ in range(2)]
         [t.start() for t in ths]; [t.join() for t in ths]
@@ -398,6 +427,8 @@ def main():
             dist.barrier()
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cv, {"resident": out_res, "e2e_pinned": out_e2e, "e2e_pageable": out_e2e_pg})
 
     st = stats[-1]
     if world > 1:

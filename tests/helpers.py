@@ -10,6 +10,14 @@ from constantine_b200.curves import CURVES  # noqa: E402
 from oracle import pyref  # noqa: E402
 
 
+def reference_c_api():
+    """The reference's typedefs and prototypes of the names our header also declares, per reference header in include order
+    (tests/golden/make_capi_golden.py)."""
+    import json
+    with open(os.path.join(ROOT, "tests", "golden", "reference_c_api.json")) as f:
+        return json.load(f)["headers"]
+
+
 def dec_point(p):
     if p is None:
         return None
